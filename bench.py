@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — rasterizer fwd+bwd Mpix/s @1080p (1M Gaussians) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -21,13 +21,17 @@ Printed (rank 0, ONE JSON line):
            / its mean launch duration measured live with CUDA events around the launch.
   cpu_baseline  the CPU oracle (oracle/sfgs_oracle.c, a port: the reference has no CPU
            path) timed on this box's host cores on a bounded sample.
+`--dump-outputs DIR` writes what the last timed step of `value` returned to its caller as DIR/<name>.npy (see
+dump_outputs); the inputs are seeded, so two builds given the same arguments can be compared output for output.
 `--impl reference` times the UNMODIFIED reference through its own stock code path: its pybind module `diff_gauss._C`
 (RAST/ext.cpp, rasterize_points.cu, cuda_rasterizer/*.cu) for `value` and its own autograd wrapper
 `diff_gauss.GaussianRasterizer` for `e2e`, installed into oracle/_ref by oracle/build_ref_torch.py; if that install is
 absent it falls back to the reference core behind the ctypes shim (oracle/_ref/libref_rasterizer.so), and to the CPU
 oracle port if nothing was built.  `reference_kind` in the line says which.
 
-Extra records in the same line (single-GPU run only; they never change `value`):
+Extra records in the same line (single-GPU run only; they never change `value`).  extra_frames, ssim and tilerows
+time K steps like the headline; knn (5 calls), train_loop (300 iterations) and next_ops (3-20 calls per op) keep
+their own fixed counts:
   extra_frames  the SURVEY 8d whole-scene orbit camera, the BASELINE configs[3] 5M-Gaussian scene and its dense variant:
                 Mpix/s, V, R and (this library) per-stage times, device-resident leg;
   ssim          fused-ssim forward(train)+backward at 1x3x1080x1920 with the 72N / 84N-byte roofline of SURVEY 8d, this
@@ -58,6 +62,7 @@ PKG = os.path.join(ROOT, "skyfall-gs_b200")
 for p in (ROOT, PKG):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True     # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -802,6 +807,37 @@ def live_traffic(kernel_regex, timeout_s=240):
             return None
 
 
+# ----------------------------------------------------------------------------- --dump-outputs
+DUMP_MAX_ELEMENTS = 1 << 20        # per array: 14 float32 arrays of <= 4 MB and radii as float64 (8 MB), ~60 MB in all
+FWD_NAMES = ("num_rendered", "color", "depth", "norm", "alpha", "radii")
+BWD_NAMES = ("grad_means2D", "grad_colors", "grad_opacity", "grad_means3D", "grad_cov3D", "grad_norm3D", "grad_sh",
+             "grad_scales", "grad_rotations")
+SHIM_BWD_KEYS = ("means2D", "colors", "opacity", "means3D", "cov3D", "norm3D", "sh", "scales", "rot")
+
+
+def dump_outputs(out, kind, path):
+    """The arrays one fwd+bwd step hands its caller: num_rendered, the four images and radii of the forward, and the
+    nine gradient tensors of the backward (the forward's opaque scratch buffers are left out).  Floating arrays are
+    written as float32, integer ones as float64.  An array of more than DUMP_MAX_ELEMENTS elements is written as a
+    sample: the elements at DUMP_MAX_ELEMENTS flat indices drawn without replacement by numpy's default_rng(0), in
+    increasing order — the same indices for every run of the same shape."""
+    f, g = out
+    if kind == "shim":
+        fwd = [f[k] for k in FWD_NAMES]
+        bwd = [g[k] for k in SHIM_BWD_KEYS]
+    else:
+        fwd, bwd = list(f[:6]), list(g[:9])
+    os.makedirs(path, exist_ok=True)
+    for name, t in zip(FWD_NAMES + BWD_NAMES, fwd + bwd):
+        t = torch.as_tensor(t).detach().reshape(-1)
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMENTS, replace=False))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        a = a.astype(np.float32) if a.dtype.kind == "f" else a.astype(np.float64)
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------- main
 def main():
     ap = argparse.ArgumentParser()
@@ -814,6 +850,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-clocks", action="store_true", help="do not sample SM clocks during the timed region")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra frames / ssim / ncu / tile-row records")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     steps, warmup = max(1, args.steps), max(3, args.warmup)
 
@@ -848,6 +885,13 @@ def main():
         step = lambda: step_ref_stock(d, cam)  # noqa: E731
     else:
         step = lambda: step_ref(d, cam)   # noqa: E731
+    last = {}
+    if args.dump_outputs:
+        timed_step = step
+
+        def step():
+            last["out"] = timed_step()
+            return last["out"]
 
     # ---- value: device-resident inputs, per-step events, max over ranks
     sampler = ClockSampler(local_rank, dev)
@@ -857,6 +901,8 @@ def main():
     ms, value_info = measure(step, steps, warmup, flush, dev,
                              between=sampler.sample if (args.impl == "ours" and not args.no_clocks) else None)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last.pop("out"), kind, args.dump_outputs)
     total_ms = torch.tensor([sum(ms)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.barrier()
@@ -889,7 +935,7 @@ def main():
         for label, P_t, extent in (("1M", P_GAUSS, 256.0), ("configs3_5M", 5_000_000, 256.0 * 5 ** 0.5)):
             try:
                 tsamp = ClockSampler(local_rank, dev)
-                rec = multigpu.run_tilerows(P_t, extent, rank, world, dev, max(10, steps), warmup)
+                rec = multigpu.run_tilerows(P_t, extent, rank, world, dev, steps, warmup)
                 tsamp.sample()
                 rec["clocks"] = tsamp.stop()
                 rec["label"] = label
@@ -982,12 +1028,12 @@ def main():
         frames = []
         for name in EXTRA_FRAMES:
             try:
-                frames.append(frame_record(name, kind, dev, max(10, steps // 2)))
+                frames.append(frame_record(name, kind, dev, steps))
             except Exception as exc:  # noqa: BLE001
                 frames.append({"name": name, "error": f"{type(exc).__name__}: {exc}"[:300]})
         out["extra_frames"] = frames
         try:
-            out["ssim"] = ssim_record(kind, dev)
+            out["ssim"] = ssim_record(kind, dev, steps)
         except Exception as exc:  # noqa: BLE001
             out["ssim"] = {"error": f"{type(exc).__name__}: {exc}"[:300]}
         try:

@@ -100,13 +100,14 @@ def backward_f64(I, means3D, radii, shs, scales, rotations, scale_modifier, view
 GRAD_KEYS = ("means2D", "colors", "opacity", "means3D", "cov3D", "norm3D", "sh", "scales", "rot")
 
 
-def error_report(ours, ref, f64, keys=GRAD_KEYS):
+def error_report(ours, ref, f64, keys=GRAD_KEYS, ref_stats=None):
     """Per tensor: the error of `ours` and of `ref` against the float64 adjudicator, as max / 99.9th percentile /
     mean / rms of the absolute error.  `ref` may be a list of runs of the reference CUDA build (its float atomics make
     it non-deterministic): every statistic is then the largest over the runs.  `ours` may be a list of runs too (its
     vector reductions are unordered as well): mean / p99.9 / rms are then the LARGEST over the runs, and the worst
     element — an extreme-value statistic whose single draws scatter by a factor of five between runs of either
-    implementation — the MEDIAN over the runs (every run's value is kept in `ours_max_runs`)."""
+    implementation — the MEDIAN over the runs (every run's value is kept in `ours_max_runs`).
+    `ref_stats` ({tensor: statistics}, from `reference_stats` of an earlier run) stands in for `ref` where given."""
     refs = [] if ref is None else (list(ref) if isinstance(ref, (list, tuple)) else [ref])
     ours_runs = list(ours) if isinstance(ours, (list, tuple)) else [ours]
 
@@ -133,9 +134,17 @@ def error_report(ours, ref, f64, keys=GRAD_KEYS):
         for r in refs:
             s1 = stats((r[k].double().flatten() - t).abs())
             sr = s1 if sr is None else {m: max(sr[m], s1[m]) for m in s1}
+        if ref_stats is not None:
+            sr = ref_stats[k]
         rep[k] = dict(ours=so, ref=sr, scale=float(t.abs().max()), n=int(t.numel()), ref_runs=len(refs),
                       ours_runs=len(runs), ours_max_runs=[r_["max"] for r_ in runs])
     return rep
+
+
+def reference_stats(ref, f64, keys=GRAD_KEYS):
+    """{tensor: error statistics of the reference runs `ref` against `f64`} — the `ref` half of error_report."""
+    rep = error_report(ref, ref, f64, keys)
+    return {k: r["ref"] for k, r in rep.items()}
 
 
 def format_report(rep) -> str:

@@ -3,7 +3,7 @@
 Not imported by the product (skyfall-gs_b200/); only tests/ use it.  Each function restates, statement by statement and
 with the same torch calls (so that it computes what the reference computes on whichever device it runs on), the
 reference code it cites.  Pinned against the reference's own GaussianModel by tests/golden/make_densify_golden.py
-(fixture tests/golden/densify_ref.npz, checked in tests/test_densify.py).
+(fixture tests/golden/densify_ref-*.npz, checked in tests/test_densify.py).
 """
 import torch
 

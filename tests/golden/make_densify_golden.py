@@ -143,8 +143,10 @@ def main():
             out[f"{case}_after_max_radii2D"] = pc.max_radii2D.numpy().copy()
             print(case, "P", P, "->", pc.get_xyz.shape[0], "counts (cloned, split, pruned)", counts, "noise", tuple(rec[0].shape))
     out["meta"] = np.array([EXTENT, MAX_GRAD, 0.005, OPT.percent_dense])
-    np.savez_compressed(os.path.join(HERE, "densify_ref.npz"), **out)
-    print("wrote densify_ref.npz")
+    sys.path.insert(0, os.path.join(HERE, ".."))
+    import golden_io
+    golden_io.save("densify_ref", out, HERE)
+    print("wrote densify_ref")
 
 
 if __name__ == "__main__":

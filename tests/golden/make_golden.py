@@ -1,8 +1,8 @@
 """Generate tests/golden/*.npz from the UNMODIFIED reference CUDA rasterizer (oracle/_ref) on a B200.
 
 Run on the GPU box (the reference cannot execute in the CPU-only container):
-    gpurun -- 'python tests/golden/make_golden.py gpurun_out/golden'
-then copy gpurun_out/golden/*.npz into tests/golden/.  The fixtures pin the CPU oracle
+    python tests/golden/make_golden.py OUT_DIR
+then copy OUT_DIR/*.npz into tests/golden/.  The fixtures pin the CPU oracle
 (tests/test_oracle_golden.py, no GPU needed) and are checked again against the product on the GPU.
 Inputs are not stored: they are regenerated from the seeds with sfgs.synthetic (numpy PCG64).
 """
@@ -15,6 +15,7 @@ for p in (ROOT, os.path.join(ROOT, "skyfall-gs_b200"), os.path.join(ROOT, "tests
 import numpy as np
 import torch
 
+import golden_io
 import helpers as Hh
 from golden_cases import CASES, build_case
 from oracle import ref_cuda
@@ -47,10 +48,11 @@ def main(out_dir):
         for k in ("means2D", "colors", "opacity", "means3D", "cov3D", "norm3D", "sh", "scales", "rot", "conic", "depths"):
             out["grad_" + k] = g[k].cpu().numpy()
             out["gradspread_" + k] = np.float32((g[k] - g2[k]).abs().max().item() if g[k].numel() else 0.0)
-        path = os.path.join(out_dir, f"ref_{name}.npz")
-        np.savez_compressed(path, **out)
-        print(name, "R=", f["num_rendered"], "visible=", int((f["radii"] > 0).sum()), os.path.getsize(path), "bytes")
+        paths = golden_io.save(f"ref_{name}", out, out_dir)
+        print(name, "R=", f["num_rendered"], "visible=", int((f["radii"] > 0).sum()), [os.path.getsize(p) for p in paths], "bytes")
 
 
 if __name__ == "__main__":
-    main(sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, "gpurun_out", "golden"))
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    main(sys.argv[1])

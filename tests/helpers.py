@@ -120,7 +120,7 @@ ADJ_FLOOR = 1e-5      # north_star: 1e-5 abs on gradient tensors
 
 
 def adjudicate_gradients(d, cam, sh_degree, bg, I, out_alpha, radii, cot, ours, ref, tag, kernel_size=0.1,
-                         scale_modifier=1.0, colors=None, factors=None, floor=ADJ_FLOOR):
+                         scale_modifier=1.0, colors=None, factors=None, floor=ADJ_FLOOR, ref_stats=None):
     """The gradient gate of the parity tests.
 
     The reference's backward is itself an approximation (float atomics in a run-dependent order, transmittance
@@ -131,7 +131,8 @@ def adjudicate_gradients(d, cam, sh_degree, bg, I, out_alpha, radii, cot, ours, 
     in the mean, at the 99.9th percentile and in the worst element.  No element is exempt.
 
     I: forward intermediates in the reference's vocabulary (oracle.ref_cuda.internals or helpers.our_internals).
-    ref: one run of the reference's gradients, or a list of runs (every statistic: the largest over the runs).
+    ref: one run of the reference's gradients, or a list of runs (every statistic: the largest over the runs); or None
+    with `ref_stats`, the reference's statistics as stored by tests/golden/make_parity_golden.py.
     ours: one run of this library's gradients, or a list of runs (mean / p99.9: the largest over the runs; the worst
     element: the median over the runs — see oracle.adjudicator.error_report).
     Returns the report (also appended to gpurun_out/adjudication.jsonl when that directory exists)."""
@@ -143,7 +144,7 @@ def adjudicate_gradients(d, cam, sh_degree, bg, I, out_alpha, radii, cot, ours, 
                          d["viewmatrix"], d["projmatrix"], d["campos"], cam.tanfovx, cam.tanfovy, kernel_size,
                          sh_degree, bg, out_alpha, cot, colors_precomp=colors)
     keys = [k for k in A.GRAD_KEYS if not (colors is not None and k == "sh")]
-    rep = A.error_report(ours, ref, f64, keys)
+    rep = A.error_report(ours, ref, f64, keys, ref_stats=ref_stats)
     print(f"\n[adjudication] {tag}\n" + A.format_report(rep))
     out_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "gpurun_out")
     if os.path.isdir(out_dir):

@@ -1,6 +1,6 @@
 """SURVEY.md 8f rank 2 — the appearance path (EmbeddingModel MLP + tone map + eval_sh -> colors_precomp).
 
-Golden vectors: tests/golden/appearance_ref.npz, produced by the reference's OWN EmbeddingModel and eval_sh
+Golden vectors: tests/golden/appearance_ref-*.npz, produced by the reference's OWN EmbeddingModel and eval_sh
 (tests/golden/make_appearance_golden.py, float32 and float64).
   * CPU: the torch formulation in sfgs/appearance.py (used for the backward pass) equals the reference modules' output;
   * GPU: the tcgen05 kernel equals it within the stated bf16 tolerance, for every SH degree, ragged P, and the
@@ -12,12 +12,14 @@ import numpy as np
 import pytest
 import torch
 
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "appearance_ref.npz")
+import golden_io
+
+
 COLOR_ATOL = 1e-4      # split-bf16 (hi + lo) tensor-core operands, fp32 accumulation: ~2^-16 relative per product
 
 
 def _load(dev, dtype=torch.float32):
-    g = np.load(GOLD)
+    g = golden_io.load("appearance_ref")
     t = {k: torch.from_numpy(g[k]).to(dev) for k in ("features", "gemb", "aemb", "xyz", "campos", "W1", "b1", "W2", "b2", "W3", "b3")}
     return g, {k: v.to(dtype) for k, v in t.items()}
 

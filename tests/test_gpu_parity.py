@@ -1,7 +1,8 @@
 """GPU parity tests (run with `-m gpu` on a B200): the CUDA path through the C ABI against
-  (1) the unmodified reference CUDA rasterizer (oracle/_ref) — bit-exact tile/key indexing, 1e-5 images,
-      gradients adjudicated by a float64 evaluation of the reference's algorithm (helpers.adjudicate_gradients:
-      our error against float64 <= 2x the reference build's own error + 1e-5, every element, no outlier budget),
+  (1) the unmodified reference CUDA rasterizer, through its results stored by tests/golden/make_parity_golden.py
+      (tests/parity_golden.py) — bit-exact tile/key indexing, 1e-5 images, gradients adjudicated by a float64
+      evaluation of the reference's algorithm (helpers.adjudicate_gradients: our error against float64 <= 2x the
+      reference build's own error + 1e-5, every element, no outlier budget),
   (2) the CPU oracle (oracle/sfgs_oracle.c),
   (3) the committed golden fixtures produced by the reference on a B200 (tests/golden/ref_*.npz),
 plus edge cases and size-independent properties at the BASELINE.json full size.
@@ -12,7 +13,10 @@ import numpy as np
 import pytest
 import torch
 
+import golden_io
 import helpers as Hh
+import parity_cases as PC
+import parity_golden as PG
 from golden_cases import CASES, build_case
 from sfgs import synthetic as S
 
@@ -26,76 +30,64 @@ def ref_available():
     return ref_cuda.available()
 
 
-def bits(t):
-    return t.contiguous().view(torch.int32) if t.dtype.is_floating_point else t
+INDEXING = ("num_rendered", "radii", "tiles_touched", "depths", "means2D", "cov3D", "conic_opacity", "ranges",
+            "point_list", "keys", "n_contrib")
 
 
-def run_pair(scene, cam, dev, bg=(0.1, 0.2, 0.3), colors=None, **kw):
-    d = Hh.to_torch(scene, cam, dev)
-    bg_t = torch.tensor(bg, device=dev, dtype=torch.float32)
-    col = None if colors is None else torch.from_numpy(colors).to(dev)
-    sh_degree = kw.pop("sh_degree", scene.sh_degree)
-    ours = Hh.run_ours_forward(d, cam, sh_degree, bg_t, colors=col, **kw)
-    ref = Hh.run_ref_forward(d, cam, sh_degree, bg_t, colors=col, **kw)
-    return d, bg_t, col, ours, ref
+class Ours:
+    """This library on one of tests/parity_cases.py's scenes, next to the reference's stored results for it."""
+
+    def __init__(self, family, cid, dev):
+        self.case = c = PC.build(family, cid)
+        self.gold = PG.load("parity_" + family, cid)
+        self.scene, self.cam, self.kw, self.dev = c.scene, c.cam, c.kw, dev
+        self.d = Hh.to_torch(c.scene, c.cam, dev)
+        self.bg = torch.tensor(c.bg, device=dev, dtype=torch.float32)
+        self.col = None if c.colors is None else torch.from_numpy(c.colors).to(dev)
+        self.fwd = self.forward()
+        P, H, W = c.scene.P, c.cam.height, c.cam.width
+        self.I = PG.ours_vocabulary(Hh.our_internals(self.fwd, P, H, W))
+        self.rec = PG.record(self.fwd, self.I, P, H, W)
+
+    def forward(self):
+        return Hh.run_ours_forward(self.d, self.cam, self.kw["sh_degree"], self.bg, kernel_size=self.kw["kernel_size"],
+                                   scale_modifier=self.kw["scale_modifier"], colors=self.col)
+
+    def check(self, fields, img_atol=IMG_ATOL, exact_images=()):
+        PG.check(self.rec, self.gold, fields, img_atol=img_atol, exact_images=exact_images)
+
+    def adjudicate(self, tag):
+        """Gradients of three runs against the float64 evaluation, next to the reference's stored statistics.
+
+        The float64 evaluation is fed this library's forward intermediates, so they are first asserted bit-identical to
+        the reference's (the blend lists, every per-Gaussian quantity the evaluation reads, and the alpha image): it
+        then computes exactly what it computes from the reference's, and an error in them cannot cancel out of the
+        comparison."""
+        self.check(("num_rendered", "radii", "ranges", "point_list", "n_contrib", "depths", "means2D", "cov3D",
+                    "conic_opacity", "norm3D") + (("rgb", "clamped") if self.col is None else ()), img_atol=None,
+                   exact_images=("alpha",))
+        cot = [torch.from_numpy(c).to(self.dev) for c in S.cotangents(self.cam.width, self.cam.height, seed=self.case.cot_seed)]
+        kw = dict(kernel_size=self.kw["kernel_size"], scale_modifier=self.kw["scale_modifier"], colors=self.col)
+        gbs = [Hh.run_ours_backward(self.d, self.cam, self.kw["sh_degree"], self.bg, self.fwd, cot, **kw)
+               for _ in range(3)]     # this library's reductions are unordered too
+        Hh.adjudicate_gradients(self.d, self.cam, self.kw["sh_degree"], self.bg, self.I, self.fwd["alpha"],
+                                self.fwd["radii"], cot, gbs, None, tag, ref_stats=PG.ref_stats(self.gold), **kw)
+        return gbs[0]
 
 
-@pytest.mark.parametrize("case", ["blob", "city", "precomp", "modifier"])
+@pytest.mark.parametrize("case", PC.FAMILIES["indexing"])
 def test_forward_bit_exact_indexing_vs_reference(cuda_device, case):
-    if not ref_available():
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_cuda
-    dev = cuda_device
-    kw, colors = {}, None
-    if case == "blob":
-        scene, cam = S.blob_scene(6000, seed=21), S.simple_camera(333, 217)
-    elif case == "city":
-        scene, cam = S.city_scene(200_000, seed=2), S.jax004_camera(1920, 1080)
-    elif case == "precomp":
-        scene, cam = S.blob_scene(3000, seed=22, sh_degree=0), S.simple_camera(256, 256)
-        colors = np.random.default_rng(0).uniform(0, 1, (scene.P, 3)).astype(np.float32)
-    else:
-        scene, cam = S.blob_scene(3000, seed=23), S.simple_camera(200, 120)
-        kw = dict(kernel_size=0.3, scale_modifier=1.7, sh_degree=2)
-    d, bg_t, col, ours, ref = run_pair(scene, cam, dev, colors=colors, **kw)
-    P, H, W = scene.P, cam.height, cam.width
-    assert ours["num_rendered"] == ref["num_rendered"]
-    assert torch.equal(ours["radii"], ref["radii"])
-    oi, ri = Hh.our_internals(ours, P, H, W), ref_cuda.internals(ref, P, H, W)
-    vis = ref["radii"] > 0
-    assert torch.equal(oi["tiles_touched"], ri["tiles_touched"])
-    for k in ("depths", "means2D", "cov3D", "conic_opacity"):
-        assert torch.equal(bits(oi[k][vis]), bits(ri[k][vis])), k
-    assert torch.equal(oi["ranges"], ri["ranges"])
-    assert torch.equal(oi["point_list"], ri["point_list"])
-    assert torch.equal(Hh.ref_style_keys(oi["ranges"], oi["keys"]), ri["keys"])
-    assert torch.equal(oi["n_contrib"], ri["n_contrib"])
-    if colors is None:
-        assert torch.equal(bits(oi["rgb"][vis]), bits(ri["rgb"][vis]))     # colours, hence clamp flags, bit for bit
-    for k in ("color", "depth", "norm", "alpha"):
-        assert (ours[k] - ref[k]).abs().max().item() <= IMG_ATOL, k
+    o = Ours("indexing", case, cuda_device)
+    # colours, hence clamp flags, bit for bit
+    o.check(INDEXING + (("rgb",) if o.col is None else ()))
 
 
-@pytest.mark.parametrize("case", ["blob", "city"])
+@pytest.mark.parametrize("case", PC.FAMILIES["backward"])
 def test_backward_vs_reference_adjudicated_by_float64(cuda_device, case):
-    if not ref_available():
-        pytest.skip("oracle/_ref not built")
-    dev = cuda_device
-    if case == "blob":
-        scene, cam = S.blob_scene(6000, seed=31), S.simple_camera(320, 200)
-    else:
-        scene, cam = S.city_scene(300_000, seed=3), S.jax004_camera(1920, 1080)
-    d, bg_t, col, ours, ref = run_pair(scene, cam, dev)
-    cot = [torch.from_numpy(c).to(dev) for c in S.cotangents(cam.width, cam.height, seed=4)]
-    from oracle import ref_cuda
-    gb = Hh.run_ours_backward(d, cam, scene.sh_degree, bg_t, ours, cot)
-    gbs = [gb] + [Hh.run_ours_backward(d, cam, scene.sh_degree, bg_t, ours, cot) for _ in range(2)]     # this library's reductions are unordered too
-    r1 = [Hh.run_ref_backward(d, cam, scene.sh_degree, bg_t, ref, cot) for _ in range(3)]
-    ri = ref_cuda.internals(ref, scene.P, cam.height, cam.width)
-    Hh.adjudicate_gradients(d, cam, scene.sh_degree, bg_t, ri, ref["alpha"], ref["radii"], cot, gbs, r1,
-                            f"backward_vs_reference[{case}]")
+    o = Ours("backward", case, cuda_device)
+    gb = o.adjudicate(f"backward_vs_reference[{case}]")
     # culled Gaussians get exact zeros
-    inv = ours["radii"] == 0
+    inv = o.fwd["radii"] == 0
     for k in ("means2D", "opacity", "means3D", "sh", "scales", "rot"):
         assert gb[k][inv].abs().max().item() == 0.0 if inv.any() else True
 
@@ -105,41 +97,16 @@ def test_randomised_differential_vs_reference(cuda_device, seed):
     """Seeded random configurations (image sizes off the tile grid, every SH degree, scale modifiers, filter sizes,
     backgrounds, cluster tightness) against the unmodified reference CUDA rasterizer: indexing bit-exact, images
     within 1e-5, gradients adjudicated by the float64 evaluation (helpers.adjudicate_gradients)."""
-    if not ref_available():
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_cuda
-    dev = cuda_device
-    rng = np.random.default_rng(1000 + seed)
-    P = int(rng.integers(1, 5000))
-    W, H = int(rng.integers(17, 400)), int(rng.integers(17, 300))
-    deg = int(rng.integers(0, 4))
-    scene = S.blob_scene(P, seed=200 + seed, sh_degree=3, spread=float(rng.uniform(0.2, 3.0)),
-                         scale=float(rng.uniform(0.01, 0.4)))
-    cam = S.simple_camera(W, H, fov_deg=float(rng.uniform(30, 90)), distance=float(rng.uniform(3.0, 10.0)))
-    kw = dict(kernel_size=float(rng.choice([0.05, 0.1, 0.3])), scale_modifier=float(rng.uniform(0.5, 2.0)), sh_degree=deg)
-    bg = tuple(float(x) for x in rng.uniform(0, 1, 3))
-    d, bg_t, col, ours, ref = run_pair(scene, cam, dev, bg=bg, **kw)
-    assert ours["num_rendered"] == ref["num_rendered"] and torch.equal(ours["radii"], ref["radii"])
-    oi, ri = Hh.our_internals(ours, P, H, W), ref_cuda.internals(ref, P, H, W)
-    assert torch.equal(oi["ranges"], ri["ranges"]) and torch.equal(oi["point_list"], ri["point_list"])
-    assert torch.equal(oi["n_contrib"], ri["n_contrib"])
-    for k in ("color", "depth", "norm", "alpha"):
-        assert (ours[k] - ref[k]).abs().max().item() <= IMG_ATOL, k
-    cot = [torch.from_numpy(c).to(dev) for c in S.cotangents(W, H, seed=seed)]
-    gb = Hh.run_ours_backward(d, cam, deg, bg_t, ours, cot, kernel_size=kw["kernel_size"], scale_modifier=kw["scale_modifier"])
-    gbs = [gb] + [Hh.run_ours_backward(d, cam, deg, bg_t, ours, cot, kernel_size=kw["kernel_size"], scale_modifier=kw["scale_modifier"]) for _ in range(2)]     # this library's reductions are unordered too
-    r1 = [Hh.run_ref_backward(d, cam, deg, bg_t, ref, cot, kernel_size=kw["kernel_size"],
-                              scale_modifier=kw["scale_modifier"]) for _ in range(3)]
-    Hh.adjudicate_gradients(d, cam, deg, bg_t, ri, ref["alpha"], ref["radii"], cot, gbs, r1, f"randomised[{seed}]",
-                            kernel_size=kw["kernel_size"], scale_modifier=kw["scale_modifier"])
+    o = Ours("random", str(seed), cuda_device)
+    o.check(("num_rendered", "radii", "ranges", "point_list", "n_contrib"))
+    o.adjudicate(f"randomised[{seed}]")
 
 
 @pytest.mark.parametrize("name", CASES)
 def test_against_golden_fixtures(cuda_device, name):
-    path = os.path.join(GOLD, f"ref_{name}.npz")
-    if not os.path.exists(path):
+    if not golden_io.exists(f"ref_{name}"):
         pytest.skip("golden fixture not generated yet")
-    g = np.load(path)
+    g = golden_io.load(f"ref_{name}")
     dev = cuda_device
     scene, cam, bg, kw = build_case(name)
     d = Hh.to_torch(scene, cam, dev)
@@ -242,60 +209,29 @@ def test_edge_cases(cuda_device):
 
 def test_long_tile_lists_use_both_sort_paths(cuda_device):
     """> 1024 and > 4096 instances in one tile exercise the heavy sort window and the global radix fallback."""
-    if not ref_available():
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_cuda
     dev = cuda_device
-    scene, cam = S.blob_scene(9000, seed=77, spread=0.25, scale=0.05), S.simple_camera(64, 64, distance=10.0)
-    d, bg_t, col, ours, ref = run_pair(scene, cam, dev, bg=(0, 0, 0))
-    oi, ri = Hh.our_internals(ours, scene.P, 64, 64), ref_cuda.internals(ref, scene.P, 64, 64)
-    longest = int((ri["ranges"][:, 1] - ri["ranges"][:, 0]).max())
+    o = Ours("long", "long", dev)
+    longest = int(o.gold["longest"])
     assert longest > 4096, longest
-    assert torch.equal(oi["point_list"], ri["point_list"]) and torch.equal(oi["ranges"], ri["ranges"])
-    assert torch.equal(oi["n_contrib"], ri["n_contrib"])
-    assert (ours["color"] - ref["color"]).abs().max().item() <= IMG_ATOL
+    o.check(("point_list", "ranges", "n_contrib"))
     # the oversized-tile path (single-CTA radix sort through global memory) must stay in the same league as the
-    # reference's global radix sort on the same frame, not fall off a cliff
-    def timed(fn):
-        for _ in range(3):
-            fn()
-        torch.cuda.synchronize(dev)
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        a.record()
-        for _ in range(10):
-            fn()
-        b.record()
-        torch.cuda.synchronize(dev)
-        return a.elapsed_time(b) / 10
-    t_ours = timed(lambda: Hh.run_ours_forward(d, cam, 3, bg_t))
-    t_ref = timed(lambda: Hh.run_ref_forward(d, cam, 3, bg_t))
+    # reference's global radix sort on the same frame (its forward time, stored with its results), not fall off a cliff
+    t_ours = PG.timed(o.forward, dev)
+    t_ref = float(o.gold["forward_ms"])
     print(f"\n[long tile lists] longest {longest}: forward {t_ours:.3f} ms (reference {t_ref:.3f} ms)")
     assert t_ours <= 1.5 * t_ref + 0.2, (t_ours, t_ref)
 
 
-@pytest.mark.parametrize("n", [1, 2, 31, 33, 127, 128, 129, 255, 256, 257, 511, 512, 513, 1023, 1024, 1025, 4095, 4096, 4097])
+@pytest.mark.parametrize("n", PC.SORT_SIZES)
 def test_sort_class_boundaries_and_depth_ties(cuda_device, n):
     """ONE tile (a 16x16 image) whose list has exactly `n` instances, at every size-class boundary of the per-tile sort:
     warp class with 4 / 8 / 16 keys per lane (<= 128 / 256 / 512), CTA class with 4 / 16 keys per thread (<= 1024 / 4096),
     global radix beyond.  A third of the Gaussians are exact duplicates of others (what densification's clone step
     produces): equal depths, so the order inside the tile is decided by the Gaussian id exactly like the reference's stable
     radix sort decides it."""
-    if not ref_available():
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_cuda
-    dev = cuda_device
-    scene = S.blob_scene(n, seed=1000 + n, spread=0.05, scale=0.08)
-    dup = np.arange(n) % 3 == 2
-    scene.means3D[dup] = scene.means3D[np.maximum(np.flatnonzero(dup) - 1, 0)]      # exact copies: depth ties
-    cam = S.simple_camera(16, 16, distance=6.0)
-    d, bg_t, col, ours, ref = run_pair(scene, cam, dev, bg=(0, 0, 0))
-    oi, ri = Hh.our_internals(ours, scene.P, 16, 16), ref_cuda.internals(ref, scene.P, 16, 16)
-    assert int(ri["ranges"][0, 1] - ri["ranges"][0, 0]) == n == int(ref["num_rendered"]) == int(ours["num_rendered"])
-    assert torch.equal(oi["ranges"], ri["ranges"])
-    assert torch.equal(oi["point_list"][:n], ri["point_list"][:n])
-    assert torch.equal(oi["n_contrib"], ri["n_contrib"])
-    assert torch.equal(ours["depth"], ref["depth"]) and torch.equal(ours["alpha"], ref["alpha"])
-    assert (ours["color"] - ref["color"]).abs().max().item() <= IMG_ATOL
+    o = Ours("sort", str(n), cuda_device)
+    assert int(o.gold["longest"]) == n == int(o.gold["num_rendered"]) == int(o.fwd["num_rendered"])
+    o.check(("ranges", "point_list", "n_contrib"), exact_images=("depth", "alpha"))
 
 
 def test_unpacked_key_path_for_more_than_2p24_gaussians(cuda_device):
@@ -305,8 +241,6 @@ def test_unpacked_key_path_for_more_than_2p24_gaussians(cuda_device):
     SFGS_KEYS_PACKED=0 (small scenes through exactly that path)."""
     import subprocess
     import sys
-    if not ref_available():
-        pytest.skip("oracle/_ref not built")
     env = dict(os.environ, SFGS_KEYS_PACKED="0")
     r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-m", "gpu", "-x", "-q", "-k",
                         "indexing or boundaries or long_tile or needles"], env=env, capture_output=True, text=True,
@@ -613,55 +547,15 @@ def test_training_loop_with_all_three_ops(cuda_device):
 
 
 # ----------------------------------------------------------------------------- the configurations that are benched
-def _benched_config(name):
-    """(scene, camera) of every frame bench.py reports a number on (BASELINE.json configs[1] and configs[3], plus the
-    SURVEY 8d whole-scene orbit stress frame and the dense 5M variant the round-1 numbers were quoted on)."""
-    if name == "configs1_1M_jax004":       # bench.py's headline frame, exactly
-        return S.city_scene(1_000_000, seed=0), S.jax004_camera(1920, 1080)
-    if name == "configs1_1M_orbit":        # SURVEY 8d second camera: fov 60, radius 300, elevation 85
-        return S.city_scene(1_000_000, seed=0), S.orbit_camera(width=1920, height=1080)
-    if name == "configs3_5M_jax004":       # SURVEY 8d config 4: same generator, extent x sqrt(5)
-        return S.city_scene(5_000_000, seed=0, extent=256.0 * 5 ** 0.5), S.jax004_camera(1920, 1080)
-    if name == "dense_5M_jax004":          # 5x the density of configs[1] in the same extent (long tile lists)
-        return S.city_scene(5_000_000, seed=0), S.jax004_camera(1920, 1080)
-    raise KeyError(name)
-
-
-@pytest.mark.parametrize("name", ["configs1_1M_jax004", "configs1_1M_orbit", "configs3_5M_jax004", "dense_5M_jax004"])
+@pytest.mark.parametrize("name", PC.BENCHED)
 def test_benched_configurations_vs_reference(cuda_device, name):
     """The frames bench.py times, diffed against the unmodified reference CUDA build at full size: every indexing
     quantity bit for bit (radii, tiles_touched, depth bits / means2D / conic, ranges, point_list, keys, n_contrib),
     the four images within 1e-5, all nine gradient tensors adjudicated by the float64 evaluation."""
-    if not ref_available():
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_cuda
-    dev = cuda_device
-    scene, cam = _benched_config(name)
-    d, bg_t, col, ours, ref = run_pair(scene, cam, dev, bg=(0.0, 0.0, 0.0))
-    P, H, W = scene.P, cam.height, cam.width
-    assert ours["num_rendered"] == ref["num_rendered"]
-    assert torch.equal(ours["radii"], ref["radii"])
-    oi, ri = Hh.our_internals(ours, P, H, W), ref_cuda.internals(ref, P, H, W)
-    vis = ref["radii"] > 0
-    assert torch.equal(oi["tiles_touched"], ri["tiles_touched"])
-    for k in ("depths", "means2D", "cov3D", "conic_opacity"):
-        assert torch.equal(bits(oi[k][vis]), bits(ri[k][vis])), k
-    assert torch.equal(oi["ranges"], ri["ranges"])
-    assert torch.equal(oi["point_list"], ri["point_list"])
-    assert torch.equal(Hh.ref_style_keys(oi["ranges"], oi["keys"]), ri["keys"])
-    assert torch.equal(oi["n_contrib"], ri["n_contrib"])
-    assert torch.equal(bits(oi["rgb"][vis]), bits(ri["rgb"][vis]))         # colours, hence clamp flags, bit for bit
-    ours_clamped = torch.stack([(oi["clamped"] >> k) & 1 for k in range(3)], 1).bool()
-    assert torch.equal(ours_clamped[vis], ri["clamped"][vis].bool())
-    for k in ("color", "depth", "norm", "alpha"):
-        assert (ours[k] - ref[k]).abs().max().item() <= IMG_ATOL, k
-    del oi
-    cot = [torch.from_numpy(c).to(dev) for c in S.cotangents(W, H, seed=1)]      # bench.py's cotangents
-    gb = Hh.run_ours_backward(d, cam, scene.sh_degree, bg_t, ours, cot)
-    gbs = [gb] + [Hh.run_ours_backward(d, cam, scene.sh_degree, bg_t, ours, cot) for _ in range(2)]     # this library's reductions are unordered too
-    r1 = [Hh.run_ref_backward(d, cam, scene.sh_degree, bg_t, ref, cot) for _ in range(3)]
-    Hh.adjudicate_gradients(d, cam, scene.sh_degree, bg_t, ri, ref["alpha"], ref["radii"], cot, gbs, r1, name)
-    inv = ours["radii"] == 0
+    o = Ours("benched", name, cuda_device)
+    o.check(INDEXING + ("rgb", "clamped"))          # colours, hence clamp flags, bit for bit
+    gb = o.adjudicate(name)
+    inv = o.fwd["radii"] == 0
     for k in ("means2D", "opacity", "means3D", "sh", "scales", "rot"):
         assert gb[k][inv].abs().max().item() == 0.0, k       # culled Gaussians get exact zeros
 
@@ -670,32 +564,11 @@ def test_long_thin_splats_crossing_many_tiles(cuda_device):
     """Needle-shaped splats (axis ratio up to 1:1000) hundreds of pixels long: the quadratic form of the conic
     cancels heavily far from the centre, which is where a block-level reach test could disagree with the reference's
     per-pixel `alpha < 1/255` test.  Indexing incl. n_contrib bit for bit, images 1e-5, gradients adjudicated."""
-    if not ref_available():
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_cuda
-    dev = cuda_device
-    rng = np.random.default_rng(7)
-    scene = S.blob_scene(4000, seed=91, spread=2.0, scale=0.02)
-    scene.scales[:, 0] = np.exp(rng.uniform(np.log(0.5), np.log(8.0), scene.P)).astype(np.float32)    # long axis
-    scene.scales[:, 1] = np.exp(rng.uniform(np.log(0.002), np.log(0.02), scene.P)).astype(np.float32)  # needle
-    scene.scales[:, 2] = scene.scales[:, 1]
-    scene.opacities[:] = rng.uniform(0.004, 1.0, (scene.P, 1)).astype(np.float32)   # includes values near 1/255
-    scene.opacities[::97] = np.float32(1.0) / np.float32(255.0)                      # exactly the threshold
-    cam = S.simple_camera(640, 400, fov_deg=50.0, distance=9.0)
-    for ks in (0.1, 0.0005):      # the second filter size leaves the conic nearly singular
-        d, bg_t, col, ours, ref = run_pair(scene, cam, dev, bg=(0.2, 0.1, 0.0), kernel_size=ks)
-        P, H, W = scene.P, cam.height, cam.width
-        oi, ri = Hh.our_internals(ours, P, H, W), ref_cuda.internals(ref, P, H, W)
-        assert torch.equal(oi["point_list"], ri["point_list"]) and torch.equal(oi["ranges"], ri["ranges"])
-        assert torch.equal(oi["n_contrib"], ri["n_contrib"]), f"n_contrib differs (kernel_size {ks})"
-        for k in ("color", "depth", "norm", "alpha"):
-            assert (ours[k] - ref[k]).abs().max().item() <= IMG_ATOL, (k, ks)
-        cot = [torch.from_numpy(c).to(dev) for c in S.cotangents(W, H, seed=12)]
-        gb = Hh.run_ours_backward(d, cam, 3, bg_t, ours, cot, kernel_size=ks)
-        gbs = [gb] + [Hh.run_ours_backward(d, cam, 3, bg_t, ours, cot, kernel_size=ks) for _ in range(2)]     # this library's reductions are unordered too
-        r1 = [Hh.run_ref_backward(d, cam, 3, bg_t, ref, cot, kernel_size=ks) for _ in range(3)]
-        Hh.adjudicate_gradients(d, cam, 3, bg_t, ri, ref["alpha"], ref["radii"], cot, gbs, r1, f"needles[k={ks}]",
-                                kernel_size=ks)
+    for ks in PC.NEEDLE_KERNELS:      # the second filter size leaves the conic nearly singular
+        o = Ours("needles", str(ks), cuda_device)
+        o.check(("point_list", "ranges", "n_contrib"))
+        o.adjudicate(f"needles[k={ks}]")
+        del o
 
 
 def test_alternating_frame_sizes_do_not_rerun_the_forward(cuda_device):

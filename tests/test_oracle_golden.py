@@ -7,6 +7,7 @@ import os
 import numpy as np
 import pytest
 
+import golden_io
 from golden_cases import CASES, build_case
 from oracle import cpu_oracle as O
 
@@ -19,10 +20,9 @@ def bits(a):
 
 @pytest.mark.parametrize("name", CASES)
 def test_oracle_matches_reference_cuda(name):
-    path = os.path.join(GOLD, f"ref_{name}.npz")
-    if not os.path.exists(path):
+    if not golden_io.exists(f"ref_{name}"):
         pytest.skip("fixture not generated")
-    g = np.load(path)
+    g = golden_io.load(f"ref_{name}")
     scene, cam, bg, kw = build_case(name)
     f = O.forward(scene.means3D, scene.scales, scene.rotations, scene.opacities, scene.shs, kw["sh_degree"],
                   cam.viewmatrix, cam.projmatrix, cam.campos, cam.width, cam.height, cam.tanfovx, cam.tanfovy, bg,
